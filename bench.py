@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- RGB+IR pairs/s of the yolov5l-CFTx3 two-stream forward on B200 (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--batch 32] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--batch 32] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 \
            --master-port P bench.py --gpus N --steps K --warmup W
 
@@ -17,8 +17,8 @@ Prints ONE JSON line on rank 0:
              step / time it is resident per step -- the union of the in-kernel %globaltimer spans of its launches
              inside a CUDA-graph replay (the timed mode), measured live -- against the measured sustained bf16 peak
   cpu_baseline  the reference's forward on the host cores on a bounded sample (batch-1 forwards of the same graph / size):
-             the UNMODIFIED reference's own modules when its tree -- or the copy staged into baseline/_ref by
-             oracle/stage_reference.py, which travels to the GPU box -- is importable (kind "reference"), else the
+             the UNMODIFIED reference's own modules when its tree -- or the copy staged into oracle/_ref by
+             oracle/stage_reference.py, which travels with the built tree -- is importable (kind "reference"), else the
              oracle's restatement of it (kind "port")
 --impl reference: the same CPU forward as a whole arm (fastest of 8/16/32/all host threads, measured first) -- rank 0 only.
 """
@@ -150,7 +150,7 @@ def best_thread_count(fwd, candidates=None):
 
 def cpu_forward(batch, force_port=False):
     """The reference's CPU forward of the headline graph on a seeded batch: (callable, kind, description).  `kind` is
-    "reference" when the UNMODIFIED reference's own modules run it (the tree, or its staged copy baseline/_ref --
+    "reference" when the UNMODIFIED reference's own modules run it (the tree, or its staged copy oracle/_ref --
     oracle/stage_reference.py; fused and eval as test.py:66-68 / detect_twostream.py:40-41 run them, fp32 on the CPU),
     else "port": the oracle's restatement of the same forward (oracle/cft_oracle.py)."""
     import torch
@@ -193,6 +193,22 @@ def cpu_baseline(seconds_budget=20.0, batch=1, force_port=False):
                       f"fastest of 8/16/32/{host_threads()} threads)"}
 
 
+def dump_outputs(out_dir, arrays, budget=64 << 20):
+    """Write each tensor of `arrays` as <out_dir>/<name>.npy in float32.  When they exceed `budget` bytes together, every
+    array keeps the same seeded subset of its rows (dim 1), so that two runs with the same arguments stay comparable."""
+    import numpy as np
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    total = sum(t.numel() * 4 for t in arrays.values())
+    for name, t in arrays.items():
+        t = t.detach().float().cpu()
+        if total > budget:
+            keep = max(1, t.shape[1] * budget // total)
+            idx = torch.randperm(t.shape[1], generator=torch.Generator().manual_seed(0))[:keep].sort().values
+            t = t[:, idx]
+        np.save(os.path.join(out_dir, name + ".npy"), t.numpy())
+
+
 def run_reference(args, rank):
     if rank != 0:
         return
@@ -202,11 +218,13 @@ def run_reference(args, rank):
     best_thread_count(fwd)                            # fastest of 8/16/32/all host threads; doubles as warm-up
     for _ in range(max(0, min(args.warmup, 2) - 1)):
         fwd()
-    steps = max(1, min(args.steps, 10))
+    steps = args.steps
     t0 = time.perf_counter()
     for _ in range(steps):
-        fwd()
+        z, _ = fwd()
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"z": z})
     v = b * steps / dt
     cores = torch.get_num_threads()
     line = {"impl": "reference", "metric": METRIC, "value": v, "unit": "pairs/s", "n_gpus": args.gpus, "steps": steps,
@@ -376,7 +394,7 @@ def gpu_eager_baseline(pkg, cfg, B, dev, steps=5):
     """The existing GPU path on the same device, a reported baseline beside cpu_baseline (never on the product path):
     the UNMODIFIED reference's own modules in PyTorch eager (cuDNN / cuBLAS), `attempt_load`-style fused and `.half()` as
     test.py:66-68,107 / detect_twostream.py:40-41,72 run them -- when the reference tree (or its staged copy
-    baseline/_ref, oracle/stage_reference.py) is present; else the oracle's restatement of the same op sequence with its
+    oracle/_ref, oracle/stage_reference.py) is present; else the oracle's restatement of the same op sequence with its
     tensors on the GPU (bf16, channels_last)."""
     import torch
     from oracle import cft_oracle as O
@@ -443,7 +461,12 @@ def main():
     ap.add_argument("--ncu-range", action="store_true",
                     help="after the measurements, run ONE eager step between cudaProfilerStart/Stop (for ncu "
                          "--profile-from-start off launch lists; numbers printed under ncu are never bench values)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step computed (z, float32) to DIR/z.npy; the inputs and weights are "
+                         "seeded, so runs with the same arguments can be compared output for output")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
 
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -522,12 +545,14 @@ def main():
     for st in engine.computes:
         st.wait_event(e0)
     for i in range(K):
-        engine.run_resident(i % engine.slots)
+        z_last = engine.run_resident(i % engine.slots)
     for st in engine.computes:
         cur.wait_stream(st)
     e1.record(cur)
     barrier()
     ms = e0.elapsed_time(e1)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"z": z_last})       # before later replays of the slot overwrite it
     clocks = sampler.stop() if rank == 0 else None
     t = torch.tensor([ms], device=dev, dtype=torch.float64)
     if world > 1:

@@ -7,13 +7,22 @@ assert the CPU restatement (``cft_oracle.forward``) reproduces it, and store the
 outputs plus float64 checksums of the seeded inputs/weights so the GPU box (which has no
 ``/root/reference``) can verify it regenerated the same tensors.
 
-    python oracle/make_golden.py          # writes tests/golden/*.pt
+It also stores the other things the tests compare against the reference: ``yaml.safe_load`` of the reference's x3 graph
+files (``reference_x3_yaml.json``) and a checkpoint pickled by the reference's own ``Model`` exactly as its ``train.py``
+writes one, of a width-1/64 variant of the s graph, xz-compressed so that it stays small (``ckpt_s_vedai_w64_half.pt.xz``).
+
+    python oracle/make_golden.py [name ...]    # writes only the named goldens (a case, reference_x3_yaml or
+                                               # ckpt_s_vedai_w64_half); without names, every case and both files
 """
 import importlib
+import json
+import lzma
 import os
 import sys
+from copy import deepcopy
 
 import torch
+import yaml
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
@@ -29,7 +38,19 @@ CASES = [
     ("l_flir_b1_64x64", "yolov5l_fusion_transformerx3_FLIR_aligned", 1, 64, 64, 0, 1, False),
     ("l_llvip_b1_64x96", "yolov5l_fusion_transformerx3_llvip", 1, 64, 96, 5, 6, False),
     ("x_flir_b1_64x64", "yolov5x_fusion_transformerx3_FLIR_aligned", 1, 64, 64, 0, 1, False),
+    ("s_vedai_b1_96x64", "yolov5s_fusion_transformerx3_vedai", 1, 96, 64, 11, 12, False),
+    ("s_vedai_b1_128x128", "yolov5s_fusion_transformerx3_vedai", 1, 128, 128, 19, 20, False),
 ]
+
+YAML_NAMES = ["yolov5l_fusion_transformerx3_FLIR_aligned", "yolov5l_fusion_transformerx3_llvip",
+              "yolov5s_fusion_transformerx3_vedai"]
+
+# the checkpoint: the s graph at width 1/64 (GPT d_model 8 / 8 / 16), weight seed 7
+CKPT_NAME, CKPT_WIDTH, CKPT_SEED = "yolov5s_fusion_transformerx3_vedai", 1 / 64, 7
+
+
+def checkpoint_config():
+    return dict(config.named_config(CKPT_NAME), width_multiple=CKPT_WIDTH)
 
 
 def checksum(t):
@@ -40,11 +61,40 @@ def state_checksum(sd):
     return float(sum(v.double().abs().sum() for v in sd.values()))
 
 
-def main():
+def write_yaml_configs(out_dir):
+    configs = {}
+    for name in YAML_NAMES:
+        with open(ref_shim.reference_yaml(name)) as f:
+            configs[name] = yaml.safe_load(f)
+    with open(os.path.join(out_dir, "reference_x3_yaml.json"), "w") as f:
+        json.dump(configs, f, indent=1)
+        f.write("\n")
+
+
+def write_checkpoint(yt, out_dir):
+    cfg = checkpoint_config()
+    model = yt.Model(cfg, ch=3)
+    model.load_state_dict(O.init_state(cfg, seed=CKPT_SEED), strict=True)
+    model.names = [f"cls{i}" for i in range(cfg["nc"])]
+    ckpt = {"epoch": 3, "best_fitness": 0.5, "training_results": "", "model": deepcopy(model).half(), "ema": None,
+            "updates": 0, "optimizer": None, "wandb_id": None}                       # train.py:850-857
+    path = os.path.join(out_dir, "ckpt_s_vedai_w64_half.pt.xz")
+    with lzma.open(path, "wb", preset=9) as f:
+        torch.save(ckpt, f)
+    print(f"{path}: {os.path.getsize(path)} bytes")
+
+
+def main(names):
     yt = ref_shim.import_reference()
     out_dir = os.path.join(ROOT, "tests", "golden")
     os.makedirs(out_dir, exist_ok=True)
+    if not names or "reference_x3_yaml" in names:
+        write_yaml_configs(out_dir)
+    if not names or "ckpt_s_vedai_w64_half" in names:
+        write_checkpoint(yt, out_dir)
     for name, cname, b, h, w, wseed, iseed, fused in CASES:
+        if names and name not in names:
+            continue
         cfg = config.named_config(cname)
         ypath = ref_shim.reference_yaml(cname)
         model = yt.Model(ypath if os.path.isfile(ypath) else cfg, ch=3).eval()
@@ -73,4 +123,4 @@ def main():
 
 
 if __name__ == "__main__":
-    main()
+    main(sys.argv[1:])

@@ -1,5 +1,5 @@
-"""Generate tests/golden/nms_cases.pt from the UNMODIFIED reference ``utils.general.non_max_suppression``
-(build container only; TEST INFRASTRUCTURE).
+"""Generate tests/golden/nms_cases.pt and nms_seed21_cases.pt from the UNMODIFIED reference
+``utils.general.non_max_suppression`` (build container only; TEST INFRASTRUCTURE).
 
 For each seeded case (``nms_oracle.make_predictions``) run the reference function (which calls the installed
 torchvision.ops.nms), assert the CPU restatement ``nms_oracle.non_max_suppression`` reproduces it bit for bit, and
@@ -32,12 +32,25 @@ CASES = [
     ("sparse_scene", (2, 6000, 3, 9), {"clusters": 400, "conf_lo": 0.2}, {"iou_thres": 0.3}),
 ]
 
+# one seeded batch under each branch of the keyword arguments (tests/test_nms_cpu.py)
+SEED21_CASES = [
+    ("seed21_default", (2, 2000, 3, 21), {}, {}),
+    ("seed21_multilabel", (2, 2000, 3, 21), {}, {"multi_label": True}),
+    ("seed21_agnostic_iou03", (2, 2000, 3, 21), {}, {"agnostic": True, "iou_thres": 0.3}),
+    ("seed21_classes_0", (2, 2000, 3, 21), {}, {"classes": [0]}),
+]
+
 
 def main():
     ref_shim.import_reference()
+    for file, cases in (("nms_cases.pt", CASES), ("nms_seed21_cases.pt", SEED21_CASES)):
+        write(cases, os.path.join(ROOT, "tests", "golden", file))
+
+
+def write(cases, path):
     from utils.general import non_max_suppression as ref_nms  # the reference's own function
     golden = {}
-    for name, (b, rows, nc, seed), pk, kw in CASES:
+    for name, (b, rows, nc, seed), pk, kw in cases:
         p = N.make_predictions(b, rows, nc, seed, **pk)
         ref = ref_nms(p.clone(), **kw)
         mine = N.non_max_suppression(p, **kw)
@@ -47,7 +60,6 @@ def main():
         golden[name] = {"args": (b, rows, nc, seed), "pred_kwargs": pk, "nms_kwargs": kw,
                         "input_checksum": float(p.double().sum()), "out": [r.clone() for r in ref]}
         print(f"{name}: {[tuple(r.shape) for r in ref]} oracle == reference")
-    path = os.path.join(ROOT, "tests", "golden", "nms_cases.pt")
     torch.save(golden, path)
     print("wrote", path, os.path.getsize(path), "bytes")
 

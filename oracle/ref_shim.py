@@ -3,7 +3,7 @@
 The reference's ``models/common.py:16-18`` imports matplotlib/seaborn through
 ``utils.plots``/``utils.metrics``; neither is installed.  Four empty ``sys.modules`` stubs
 make it importable (SURVEY.md §8c).  Nothing under ``/root/reference`` is modified.
-The GPU box has no ``/root/reference``: there the shim falls back to ``baseline/_ref/`` -- a git-ignored copy of the
+Where the tree itself is absent (the GPU machine) the shim falls back to ``oracle/_ref/`` -- a git-ignored copy of the
 tree's ``models/`` and ``utils/`` staged by ``oracle/stage_reference.py`` at build time (SURVEY.md §8c) -- so that the
 reference-through-the-boundary tests run on the GPU as well; they skip when neither exists.
 """
@@ -11,7 +11,7 @@ import os
 import sys
 import types
 
-_STAGED = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "baseline", "_ref")
+_STAGED = os.path.join(os.path.dirname(os.path.abspath(__file__)), "_ref")
 REF_ROOT = os.environ.get("CFT_REFERENCE_ROOT") or (
     "/root/reference" if os.path.isfile("/root/reference/models/yolo_test.py") else _STAGED)
 

@@ -7,7 +7,7 @@ model, `ComputeLoss` of `utils/loss.py:88-216`, backward, SGD + nesterov `train.
            scripts/train_step.py [--batch 32] [--steps 6] [--warmup 2] [--cfg yolov5l_fusion_transformerx3_FLIR_aligned]
 
 What runs where.  The model, the loss and the backward are the UNMODIFIED reference's own PyTorch modules / autograd
-(from /root/reference, or its staged copy baseline/_ref on the GPU box): this repository has no backward kernels
+(from the reference tree, or its staged copy oracle/_ref on the GPU machine): this repository has no backward kernels
 (DESIGN.md section 6), and its forward kernels are eval-only (BatchNorm running statistics folded), so the train-mode
 forward is the reference's too.  What this repository contributes to the step is the one exchange of the path: the
 gradient all-reduce (`allreduce.GradientAllReduce`, NCCL over NVLink / NVSwitch).  Three variants of the same step are timed,

@@ -33,3 +33,28 @@ def test_reference_arm_prints_one_contract_line(mode):
     assert cb["value"] == d["value"] and cb["cores"] >= 1
     want = "reference" if (mode == "default" and ref_shim.available()) else "port"
     assert cb["kind"] == want, cb
+
+
+def test_reference_arm_times_every_step_and_dumps_the_last_output(tmp_path, monkeypatch):
+    """`--steps` is the number of timed forwards, and `--dump-outputs` writes what the last of them returned: the arm's
+    forward is replaced by one that counts its calls and returns a distinct z each time."""
+    import numpy as np
+    import torch
+    import bench
+    calls = []
+
+    def fwd():
+        calls.append(None)
+        return torch.full((1, 7, 8), float(len(calls))), None
+    monkeypatch.setattr(bench, "cpu_forward", lambda batch: (fwd, "port", "counting stub"))
+    monkeypatch.setattr(bench, "best_thread_count", lambda f: 1)
+    monkeypatch.setattr(sys, "argv", ["bench.py", "--impl", "reference", "--steps", "11", "--warmup", "1",
+                                      "--dump-outputs", str(tmp_path)])
+    bench.main()
+    assert len(calls) == 11                                        # warm-up 1 = the thread probe only (stubbed here)
+    z = np.load(tmp_path / "z.npy")
+    assert z.dtype == np.float32 and z.shape == (1, 7, 8) and (z == 11.0).all()
+    for steps in ("0", "-3"):
+        monkeypatch.setattr(sys, "argv", ["bench.py", "--impl", "reference", "--steps", steps])
+        with pytest.raises(SystemExit):
+            bench.main()

@@ -1,13 +1,10 @@
 """CPU suite (-m "not gpu"): the oracle against the committed golden vectors (which are outputs of the
-UNMODIFIED reference, see oracle/make_golden.py) and, when /root/reference is present, against the
-reference itself."""
+UNMODIFIED reference, see oracle/make_golden.py)."""
 import glob
 import os
 
 import pytest
 import torch
-
-from oracle import ref_shim
 
 
 def _cases(golden_dir):
@@ -35,9 +32,18 @@ def test_oracle_matches_reference_golden(name, golden_dir, cft, oracle):
     assert z.shape == g["z"].shape
     # fp32 CPU: identical op sequence -> tight; fused goldens differ by the fold's rounding only
     tol = 2e-3 if g["fused"] else 1e-4
-    assert (z - g["z"]).abs().max().item() <= tol
+    assert_close_fp32(z[..., :4], g["z"][..., :4], tol)                  # boxes, in pixels
+    assert_close_fp32(z[..., 4:], g["z"][..., 4:], tol)                  # scores
     for a, b in zip(raw, g["raw"]):
-        assert (a - b).abs().max().item() <= (1e-3 if g["fused"] else 1e-5)
+        assert_close_fp32(a, b, 1e-3 if g["fused"] else 1e-5)
+
+
+def assert_close_fp32(a, b, atol):
+    """max|a - b| <= atol + 64 fp32 eps x max|b|.  The goldens were written with 8 intra-op threads and the oracle
+    reproduces them exactly at that count; PyTorch's CPU kernels split their fp32 sums by thread count, so another count
+    (``torch.set_num_threads`` 1, 4 or 16, on the same AVX-512 host) differs by up to 26 eps of the tensor's largest value
+    in the z boxes (l_flir_b1_64x64) and 20 eps in the raw heads."""
+    assert (a - b).abs().max().item() <= atol + 64 * torch.finfo(torch.float32).eps * b.abs().max().item()
 
 
 def fuse_state(sd):
@@ -81,17 +87,19 @@ def test_flop_model(cft, oracle):
     assert abs(f(cft.named_config("yolov5l_fusion_transformerx3_llvip"), 1024, 1280) / 1e9 - 641.42) < 0.01
 
 
-@pytest.mark.skipif(not ref_shim.available(), reason="/root/reference not present (GPU box)")
-def test_oracle_equals_live_reference(cft, oracle):
-    yt = ref_shim.import_reference()
-    name = "yolov5s_fusion_transformerx3_vedai"
-    cfg = cft.named_config(name)
-    model = yt.Model(ref_shim.reference_yaml(name), ch=3).eval()
+def test_oracle_equals_stored_reference(golden_dir, cft, oracle):
+    """The reference's own eval forward (s graph, weight seed 11, input seed 12), stored by oracle/make_golden.py."""
+    g = torch.load(os.path.join(golden_dir, "s_vedai_b1_96x64.pt"))
+    assert (g["config"], g["weight_seed"], g["input_seed"], g["fused"]) == ("yolov5s_fusion_transformerx3_vedai", 11, 12, False)
+    z_ref, raw_ref = g["z"], g["raw"]
+    cfg = cft.named_config(g["config"])
     sd = oracle.init_state(cfg, seed=11)
-    model.load_state_dict(sd, strict=True)
     x, x2 = oracle.make_inputs(1, 96, 64, seed=12)
-    with torch.no_grad():
-        z_ref, raw_ref = model(x, x2)
+    assert abs(float(x.double().sum()) - g["input_checksum"][0]) < 1e-6
+    assert abs(float(x2.double().sum()) - g["input_checksum"][1]) < 1e-6
+    assert abs(float(sum(v.double().abs().sum() for v in sd.values())) - g["state_checksum"]) < 1e-3
     z, raw = oracle.forward(sd, cfg, x, x2)
-    assert (z - z_ref).abs().max().item() <= 1e-5
-    assert max((a - b).abs().max().item() for a, b in zip(raw, raw_ref)) <= 1e-6
+    assert_close_fp32(z[..., :4], z_ref[..., :4], 1e-5)
+    assert_close_fp32(z[..., 4:], z_ref[..., 4:], 1e-5)
+    for a, b in zip(raw, raw_ref):
+        assert_close_fp32(a, b, 1e-6)
