@@ -8,7 +8,7 @@
 // [c*DC, (c+1)*DC) of the residual stream (fp32, in REGISTERS for the whole kernel), the heads that live in those
 // columns, and the matching N-slices of all four Linear layers:
 //
-//   LN    row statistics: per-CTA partial sums exchanged through distributed shared memory (one cluster barrier); every
+//   LN    row statistics: per-CTA (mean, M2) exchanged through distributed shared memory (one cluster barrier); every
 //         CTA normalises its own column slice, writes it (bf16, UMMA K-major SWIZZLE_128B layout) into chunk c of its
 //         resident A operand and pushes that 16 KiB chunk into the same place of every peer with a DSMEM bulk copy that
 //         signals the peer's chunk mbarrier -- the all-gather never touches L2 and needs no second barrier
@@ -125,7 +125,7 @@ cft_gpt_block_kernel(const __grid_constant__ BlockMaps maps, const __grid_consta
   float* smax = reinterpret_cast<float*>(misc + 512);          // [4][128]  (group * 2 + half)
   float* ssum = smax + 4 * kT;                                 // [4][128]
   float2* part = reinterpret_cast<float2*>(misc + 512);            // [4][128] LayerNorm partials of the column quarters (aliases smax | ssum)
-  float2* stats = part + 4 * kT;                               // [2][C][128] per-CTA partial (sum, sum of squares)
+  float2* stats = part + 4 * kT;                               // [2][C][128] per-CTA partial (mean, M2) of its DC columns
   float* lpar = reinterpret_cast<float*>(stats + 2 * p.C * kT);  // [13 DC] this layer's biases / LN parameters of the CTA's columns
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -438,14 +438,24 @@ cft_gpt_block_kernel(const __grid_constant__ BlockMaps maps, const __grid_consta
       }
     };
     // LayerNorm of the cluster-distributed rows.  dst_f32 == null: the normalised slice becomes the next A operand.
+    // Row statistics are (mean, M2 = sum of squared deviations) at every level -- two passes over the thread's registers,
+    // then Chan's merge of equal counts, M2 = sum M2_i + n * sum (mean_i - mean)^2.  The one-pass Q / d - mean^2 cancels
+    // catastrophically in fp32 once |mean| / std passes ~10 (rstd off by 1e-3 at 100, by 10 % at 1000).
     auto ln_step = [&](const float* gamma, const float* beta, float eps, float* dst_f32, int mk) {
-      float s = 0.f, sq = 0.f;
+      float s0 = 0.f, s1 = 0.f, q0 = 0.f, q1 = 0.f;      // two independent chains per pass
 #pragma unroll
-      for (int i = 0; i < NC; ++i) {
-        s += xv[i];
-        sq = fmaf(xv[i], xv[i], sq);
+      for (int i = 0; i < NC; i += 2) {
+        s0 += xv[i];
+        s1 += xv[i + 1];
       }
-      part[qd * kT + t] = make_float2(s, sq);
+      const float m = (s0 + s1) * (1.0f / NC);
+#pragma unroll
+      for (int i = 0; i < NC; i += 2) {
+        const float e0 = xv[i] - m, e1 = xv[i + 1] - m;
+        q0 = fmaf(e0, e0, q0);
+        q1 = fmaf(e1, e1, q1);
+      }
+      part[qd * kT + t] = make_float2(m, q0 + q1);
       // gamma / beta of this thread's columns: issue the loads before the barriers
       float4 gg[NC / 4], bb[NC / 4];
 #pragma unroll
@@ -456,23 +466,29 @@ cft_gpt_block_kernel(const __grid_constant__ BlockMaps maps, const __grid_consta
       named_bar_sync(3, kCompute);
       if (qd == 0) {
         const float2 a0 = part[t], a1 = part[kT + t], a2 = part[2 * kT + t], a3 = part[3 * kT + t];
-        const float cs = (a0.x + a1.x) + (a2.x + a3.x), cq = (a0.y + a1.y) + (a2.y + a3.y);
+        const float cm = ((a0.x + a1.x) + (a2.x + a3.x)) * 0.25f;
+        const float e0 = a0.x - cm, e1 = a1.x - cm, e2 = a2.x - cm, e3 = a3.x - cm;
+        const float cq = ((a0.y + a1.y) + (a2.y + a3.y)) + static_cast<float>(NC) * ((e0 * e0 + e1 * e1) + (e2 * e2 + e3 * e3));
         const uint32_t laddr = smem_u32(&stats[(sbuf * C + rank) * kT + t]);
-        for (int r = 0; r < C; ++r) st_cluster_v2f32(mapa_u32(laddr, static_cast<uint32_t>(r)), cs, cq);
+        for (int r = 0; r < C; ++r) st_cluster_v2f32(mapa_u32(laddr, static_cast<uint32_t>(r)), cm, cq);
       }
       cb();
       mark(mk);
       if (dst_f32 == nullptr) arm_chunks();
-      float S = 0.f, Q = 0.f;
+      const float2* st = stats + sbuf * C * kT + t;
+      float S = 0.f;
+      for (int j = 0; j < C; ++j) S += st[j * kT].x;
+      const float inv_d = 1.0f / static_cast<float>(d);
+      const float mean = S * (static_cast<float>(DC) * inv_d);      // the mean of C equal-count means
+      float Q = 0.f, D = 0.f;
       for (int j = 0; j < C; ++j) {
-        const float2 v = stats[(sbuf * C + j) * kT + t];
-        S += v.x;
+        const float2 v = st[j * kT];
+        const float e = v.x - mean;
         Q += v.y;
+        D = fmaf(e, e, D);
       }
       sbuf ^= 1u;
-      const float inv_d = 1.0f / static_cast<float>(d);
-      const float mean = S * inv_d;
-      const float var = fmaxf(Q * inv_d - mean * mean, 0.f);
+      const float var = fmaf(static_cast<float>(DC), D, Q) * inv_d;
       const float rstd = rsqrtf(var + eps);
 #pragma unroll
       for (int i = 0; i < NC; i += 8) {

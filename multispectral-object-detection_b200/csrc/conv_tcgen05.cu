@@ -1017,8 +1017,9 @@ extern "C" int cft_conv2d(const cft_conv_args* a, void* stream_v) {
   p.tiles_y = (p.Ho + p.TH - 1) / p.TH;
   p.block_n = pick_block_n(a->Cout);
   const long long m_tiles = static_cast<long long>((p.B + p.TB - 1) / p.TB) * p.tiles_x * p.tiles_y;
-  // too few tiles to fill the GPU (the M = 4096 GEMMs of the CFT blocks): trade tile width for parallelism
-  while (a->Cin * p.taps <= 1024 && 2 * m_tiles * ((a->Cout + p.block_n - 1) / p.block_n) <= sm_count() &&
+  // too few tiles to fill the GPU (the M = 4096 GEMMs of the CFT blocks): trade tile width for parallelism.  Not with a
+  // chained 1x1: its second GEMM needs all Cout channels of y in one tile (n_blocks = 1)
+  while (!chain && a->Cin * p.taps <= 1024 && 2 * m_tiles * ((a->Cout + p.block_n - 1) / p.block_n) <= sm_count() &&
          p.block_n >= 128 && (p.block_n / 2) % 32 == 0 && a->Cout % (p.block_n / 2) == 0)
     p.block_n /= 2;
   p.n_blocks = (a->Cout + p.block_n - 1) / p.block_n;

@@ -111,6 +111,24 @@ def test_gpt_linear_shapes_get_valid_plans(cft):
                 _check(p, 1, 1, M, cin, cout, 1, 1, f"gemm M{M} K{cin} N{cout}")
 
 
+def test_chained_1x1_keeps_every_channel_in_one_n_block(cft):
+    """The chained 1x1 multiplies the whole Cout-wide tile of y: a layer with few tiles must not get its N split into
+    n-blocks the way an unchained one does (1x1 producers and Cin <= 113 3x3 producers of 128 channels)."""
+    L = cft._lib
+    lib = cft.load()
+    for B, H, W, cin, cout, k, s in ((3, 20, 26, 128, 128, 1, 1), (1, 1, 265, 128, 128, 1, 1), (1, 160, 160, 64, 128, 3, 2),
+                                     (3, 80, 104, 64, 128, 3, 2), (2, 32, 32, 64, 64, 3, 1), (1, 20, 20, 128, 128, 3, 1)):
+        unchained = _plan(cft, B, H, W, cin, cout, k, s)
+        a = L.ConvArgs()
+        a.x, a.w, a.y, a.w2, a.y2 = 0x100000, 0x200000, 0x300000, 0x400000, 0x500000
+        a.B, a.H, a.W, a.Cin, a.ldx = B, H, W, cin, cin
+        a.Cout, a.k, a.stride, a.act, a.act2, a.ldy, a.ldy2 = cout, k, s, 1, 1, cout, cout
+        p = L.ConvPlan()
+        assert lib.cft_debug_conv_plan(C.byref(a), C.byref(p)) == 0, lib.cft_last_error().decode()
+        what = f"{cin}->{cout} k{k}s{s} {H}x{W} B{B} (unchained block_n {unchained.block_n})"
+        assert p.n_blocks == 1 and p.block_n == cout and p.num_tiles * p.ctas >= p.m_tiles, what
+
+
 def test_plan_grid_of_shapes(cft):
     """Dense grid: every combination must either plan validly or be rejected with CFT_E_ARG -- never plan garbage."""
     L = cft._lib

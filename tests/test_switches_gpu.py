@@ -11,11 +11,14 @@ pytestmark = pytest.mark.gpu
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 KERNELS = os.path.join("tests", "test_kernels_gpu.py")
 MODEL = os.path.join("tests", "test_model_gpu.py")
+EXACT = os.path.join("tests", "test_exact_gpu.py")
 
 ARMS = [
     # environment, test file, -k filter
     ({"CFT_SILU_EXP2": "1"}, KERNELS, "conv_tcgen05 or chained"),          # SiLU as x * rcp(1 + 2^-x) instead of h + h tanh(h)
     ({"CFT_GELU_ERFF": "1"}, KERNELS, "gemm_linear"),                      # erff instead of the A&S erf-GELU
+    ({"CFT_SILU_EXP2": "1"}, EXACT, "activation"),                         # ... each within its own documented error bound
+    ({"CFT_GELU_ERFF": "1"}, EXACT, "activation"),
     ({"CFT_NO_ROW_REUSE": "1"}, KERNELS, "conv_tcgen05 or chained"),       # every 3x3 on the plain one-tap-per-stage path
     ({"CFT_NO_BRES": "1"}, KERNELS, "conv_tcgen05 or chained"),            # no resident 3x3 weights
     ({"CFT_NO_PDL": "1"}, KERNELS, "conv_tcgen05 or gemm_linear"),         # no programmatic dependent launch
@@ -30,7 +33,8 @@ ARMS = [
 ]
 
 
-@pytest.mark.parametrize("env,path,expr", ARMS, ids=["+".join(f"{k}={v}" for k, v in a[0].items()) for a in ARMS])
+@pytest.mark.parametrize("env,path,expr", ARMS, ids=["+".join(f"{k}={v}" for k, v in a[0].items()) +
+                                                     ("-exact" if a[1] == EXACT else "") for a in ARMS])
 def test_non_default_arm(env, path, expr):
     e = dict(os.environ)
     e.update(env)
