@@ -146,7 +146,11 @@ int cft_layernorm(const float* x, const float* gamma, const float* beta, float e
 
 /* Multi-head self-attention core (models/common.py:497-510): qkv bf16 [B*T, 3*C] holding
  * q|k|v (head h at columns h*dk of each third), T tokens per image (T <= 128),
- * out bf16 [B*T, C] = softmax(q k^T / sqrt(dk)) v with heads merged. */
+ * out bf16 [B*T, C] = softmax(q k^T / sqrt(dk)) v with heads merged.
+ * dk = C / heads must be a multiple of 8; qkv and out must be 16-byte aligned (CFT_E_ARG otherwise).
+ * T = 128 with 16 <= dk <= 256 runs on the tensor cores when the head dim splits into at most 4 chunks of 64 / 32 / 16
+ * (a last chunk of 16 may cover the final 8 columns); every other shape runs on a CUDA-core kernel whose shared memory
+ * (3 * 128 * (dk + 2) * 2 + 128 * 129 * 4 bytes) must stay within 220 KiB, i.e. dk <= 200 -- beyond that CFT_E_ARG. */
 int cft_attention(const void* qkv, void* out, int B, int T, int C, int heads, void* stream);
 
 /* ---------------------------------------------------------------------------------------
@@ -160,7 +164,7 @@ int cft_attention(const void* qkv, void* out, int B, int T, int C, int heads, vo
  *   ln1_*, ln2_*  f32 [layers*d] (ln_input / ln_output of every layer),  lnf_*  f32 [d]
  *   workspace: cft_gpt_block_workspace_bytes(B, d) bytes, 128-byte aligned (all-gathered bf16 operands)
  *   cluster: CTAs per image (0 = automatic);  debug_x: optional f32 [layers, B, 128, d] dump of x after each layer
- * Supported: 128 tokens, head dim 16/32/64/128, d <= 512 with d / cluster in {64, 128}
+ * Supported: 128 tokens, head dim 16/32/64, d <= 512 with d / cluster in {64, 128}
  * (cft_gpt_block_supported() tells); anything else returns CFT_E_UNSUPPORTED and the caller runs the per-op path
  * (cft_layernorm / cft_conv2d / cft_attention).
  * ------------------------------------------------------------------------------------- */

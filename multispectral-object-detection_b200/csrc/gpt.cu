@@ -446,6 +446,9 @@ extern "C" int cft_attention(const void* qkv, void* out, int B, int T, int C, in
   CFT_REQUIRE(qkv && out, "cft_attention: null pointer");
   CFT_REQUIRE(B > 0 && B <= 65535 && T > 0 && T <= 128 && heads > 0 && C % heads == 0 && (C / heads) % 8 == 0,
               "cft_attention: need T<=128 and head dim multiple of 8 (T %d C %d heads %d)", T, C, heads);
+  // both kernels move q / k / v and the output in 16-byte vectors (TMA boxes, bf16x8 loads and stores)
+  CFT_REQUIRE(reinterpret_cast<uintptr_t>(qkv) % 16 == 0 && reinterpret_cast<uintptr_t>(out) % 16 == 0,
+              "cft_attention: qkv and out must be 16-byte aligned");
   static const bool force_simt = getenv("CFT_ATTENTION_SIMT") != nullptr;   // debug / cross-check
   if (!force_simt) {
     const int rc = attention_tcgen05(qkv, out, B, T, C, heads, stream);

@@ -57,6 +57,7 @@ CASES = [
     (512, 2, 3, 4),       # the same split forced
     (128, 8, 2, 0),       # yolov5s P3: cluster 2, dk 16 (SWIZZLE_32B tiles), 4 heads per CTA = two head pairs
     (256, 1, 45, 4),      # more images than co-resident clusters: clusters loop over images
+    (256, 8, 3, 2),       # the d = 256 plan of batches 34-66: cluster 2, DC 128, dk 32, 4 heads per CTA = two head pairs
 ]
 
 

@@ -348,6 +348,8 @@ def _ln_check(y, x, gamma, beta, eps, tags, what):
     print(f"\n{what}: worst |y - ref| (ratio to the tolerance) per |mean| / std")
     for r in (*RATIOS, -1.0):
         sel = tags == r
+        if not sel.any():
+            continue
         print(f"  {'constant' if r < 0 else f'{r:g}':>8}: {float(err[sel].max()):.3e} ({float(ratio[sel].max()):.3f})")
     worst = int(ratio.argmax())
     assert float(ratio.max()) <= 1.0, (f"{what}: row with |mean|/std {float(tags[worst]):g} off by "

@@ -94,6 +94,22 @@ def test_forward_fails_loudly_without_cuda(cft):
         model(x, x)
 
 
+def test_attention_rejects_misaligned_pointers(cft):
+    """Both attention kernels move q / k / v and the output in 16-byte vectors, so cft_attention refuses a qkv or out
+    pointer that is not 16-byte aligned (CFT_E_ARG) before it touches the device.  The pointers are fake: without a
+    GPU the call can only return an error; with one, an unchecked build would dereference them."""
+    if torch.cuda.is_available():
+        pytest.skip("fake device pointers: run only where no kernel can be launched")
+    lib = cft.load()
+    good_qkv, good_out = 0x10000000, 0x20000000
+    for qkv, out in ((good_qkv + 2, good_out), (good_qkv + 8, good_out), (good_qkv, good_out + 2),
+                     (good_qkv, good_out + 8), (good_qkv + 4, good_out + 4)):
+        for T, dk in ((128, 64), (64, 8)):                              # the tcgen05 shape and a CUDA-core-only one
+            rc = lib.cft_attention(qkv, out, 2, T, 8 * dk, 8, None)
+            assert rc == 1, (hex(qkv), hex(out), T, rc)                 # CFT_E_ARG
+            assert "aligned" in lib.cft_last_error().decode()
+
+
 def test_weight_packing_folds_bn_like_reference(cft):
     """pack_conv_weight == fuse_conv_and_bn (utils/torch_utils.py:181-201) then OIHW -> [O][tap][I]."""
     from importlib import import_module

@@ -12,6 +12,7 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 KERNELS = os.path.join("tests", "test_kernels_gpu.py")
 MODEL = os.path.join("tests", "test_model_gpu.py")
 EXACT = os.path.join("tests", "test_exact_gpu.py")
+ATTENTION_EXACT = os.path.join("tests", "test_attention_exact_gpu.py")
 
 ARMS = [
     # environment, test file, -k filter
@@ -25,6 +26,7 @@ ARMS = [
     ({"CFT_CONV_CTAS": "1"}, KERNELS, "conv_tcgen05 or chained or gemm_linear"),   # never CTA pairs
     ({"CFT_CONV_CTAS": "2"}, KERNELS, "conv_tcgen05 or chained or gemm_linear"),   # CTA pairs wherever legal
     ({"CFT_ATTENTION_SIMT": "1"}, KERNELS, "attention_core"),              # the CUDA-core attention cross-check kernel
+    ({"CFT_ATTENTION_SIMT": "1"}, ATTENTION_EXACT, "per_op_attention"),    # ... bit-exact at T = 128 (P not rounded)
     ({"CFT_NO_BATCH_TILES": "1"}, KERNELS, "conv_tcgen05 or chained"),     # tiles never span images (the round-1 tiling)
     ({"CFT_NO_CONV_CHAIN": "1"}, MODEL, "golden"),                         # every Bottleneck 1x1 launched separately
     ({"CFT_NO_FUSED_BLOCK": "1"}, MODEL, "golden"),                        # CFT blocks on the per-op path
@@ -34,7 +36,8 @@ ARMS = [
 
 
 @pytest.mark.parametrize("env,path,expr", ARMS, ids=["+".join(f"{k}={v}" for k, v in a[0].items()) +
-                                                     ("-exact" if a[1] == EXACT else "") for a in ARMS])
+                                                     {EXACT: "-exact", ATTENTION_EXACT: "-attention-exact"}.get(a[1], "")
+                                                     for a in ARMS])
 def test_non_default_arm(env, path, expr):
     e = dict(os.environ)
     e.update(env)
